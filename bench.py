@@ -21,6 +21,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True      # the benchmark leaves the tree it runs from as it found it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -455,8 +456,12 @@ def main():
     ap.add_argument("--cpu-baseline-log-rows", type=int, default=18)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-replicas", action="store_true", help="N > 1: skip the independent-proofs-per-GPU figure")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (the CBOR proof, one byte per float32) to DIR/proof.npy")
     ap.add_argument("--tracegen", default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.tracegen:
         w, lr = resolve_workload(args)
         _tracegen_to_files(w, lr, args.tracegen)
@@ -577,6 +582,10 @@ def main():
     phases = vb.last_prove_phases(ctx)
     # one proof per step whatever N: rows proven = rows * steps, time = the slowest rank's
     value, ms_total_max = aggregate_throughput(dist, rows * args.steps, ms_total, device="cuda", sum_rows=False)
+    if args.dump_outputs and rank == 0:
+        # every rank of a split proof returns the same bytes; float32 holds each byte exactly
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "proof.npy"), np.frombuffer(proof, dtype=np.uint8).astype(np.float32))
 
     # ---- the same K steps again with a CUDA-event pair around every kernel launch (per-kernel roofline) ----
     ctx.set_kernel_timing(True)

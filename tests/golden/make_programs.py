@@ -1,12 +1,13 @@
 """Extracts the instruction tables of the reference's proving tests (basic/tests/test_prover.rs:190-402:
 left_imm_ops_program, signed_inequality_program, loadfp_program) and the VM-state assertions that
-follow them (test_prover.rs:490-625) into tests/golden/programs.json.  Run in the build container
-(the reference tree is not present on the GPU box):  python tests/golden/make_programs.py"""
+follow them (test_prover.rs:490-625) into tests/golden/programs.json, so that the tests need no copy of the reference:
+    python tests/golden/make_programs.py <reference checkout>"""
 import json
 import os
 import re
+import sys
 
-SRC = "/root/reference/basic/tests/test_prover.rs"
+SRC = os.path.join(sys.argv[1], "basic", "tests", "test_prover.rs")
 OPC = {"Load32": 1, "Store32": 2, "Jal": 3, "Jalv": 4, "Beq": 5, "Bne": 6, "Imm32": 7, "Stop": 8, "LoadFp": 10, "Add32": 100, "Sub32": 101,
        "Lt32": 104, "Lte32": 115, "Slt32": 117, "Sle32": 118}
 txt = open(SRC).read()
