@@ -215,6 +215,19 @@ void vgpu_tree_share(uint64_t len, int32_t nranks, int32_t rank, uint64_t* begin
 #define VGPU_REJECT_CUMULATIVE_SUM (-7)   /* LogUp sums over all chips do not cancel (derive/src/lib.rs:640-647) */
 #define VGPU_REJECT_CONSTRAINTS_CHIP0 (-100) /* chip i's constraints at zeta: -100 - i (OodEvaluationMismatch) */
 int32_t vgpu_verify(vgpu_ctx* ctx, const uint8_t* proof, uint64_t proof_len, const vgpu_matrix prep[2], int32_t repr, int32_t* verdict);
+/* Machine::verify for n proofs in one call, checked on the device.  Proof i is checked against the preprocessed traces
+ * prep[2*program_of[i]] (program ROM) and prep[2*program_of[i]+1] (range table); n_programs pairs are given and each
+ * preprocessed commitment is computed once per call.  verdicts[i] is exactly what vgpu_verify returns for proof i alone
+ * (VGPU_ACCEPT or the FIRST failed check, in vgpu_verify's order).  Decoding and the transcript replay run on host threads;
+ * the Merkle paths, reduced openings, FRI folds and constraints at zeta of all proofs run as a few kernels.  Proofs of
+ * different programs and trace heights may be mixed.  Returns 0 when the checks ran; non-zero = API / device error
+ * (vgpu_last_error).  n = 0 is valid and writes nothing. */
+int32_t vgpu_verify_batch(vgpu_ctx* ctx, const uint8_t* const* proofs, const uint64_t* proof_lens, uint32_t n,
+                          const vgpu_matrix* prep, uint32_t n_programs, const uint32_t* program_of, int32_t repr,
+                          int32_t* verdicts);
+/* Wall-clock stretches of the last vgpu_verify_batch on this context (decode, preprocessed commitments, transcripts, packing,
+ * device checks); returns the number of stretches, writes at most cap. */
+uint32_t vgpu_last_verify_batch_phases(const vgpu_ctx* ctx, const char** names, float* ms, uint32_t cap);
 
 /* ---- host witness generation (Chip::generate_trace x14; machine/src/chip.rs:22) -------------------
  * program_words: n_instr x 6 int32 (opcode, a, b, c, d, e) as ProgramROM<i32> (machine/src/program.rs:165-185). */

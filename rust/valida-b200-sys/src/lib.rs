@@ -147,6 +147,8 @@ extern "C" {
 
     // ---- Machine::verify ----
     pub fn vgpu_verify(ctx: *mut vgpu_ctx, proof: *const u8, proof_len: u64, prep: *const vgpu_matrix, repr: i32, verdict: *mut i32) -> i32;
+    pub fn vgpu_verify_batch(ctx: *mut vgpu_ctx, proofs: *const *const u8, proof_lens: *const u64, n: u32, prep: *const vgpu_matrix, n_programs: u32, program_of: *const u32, repr: i32, verdicts: *mut i32) -> i32;
+    pub fn vgpu_last_verify_batch_phases(ctx: *const vgpu_ctx, names: *mut *const c_char, ms: *mut f32, cap: u32) -> u32;
 
     // ---- witness generation (host and device) ----
     pub fn vgpu_machine_run(program_words: *const i32, n_instr: u64, initial_pc: u32, initial_fp: u32, max_cycles: u64, out: *mut *mut vgpu_traces, err: *mut c_char, err_len: u64) -> i32;

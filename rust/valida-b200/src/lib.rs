@@ -158,6 +158,22 @@ impl Context {
         Ok(if verdict == sys::VGPU_ACCEPT { Verdict::Accept } else { Verdict::Reject(verdict) })
     }
 
+    /// `Machine::verify` for many proofs in one call, checked on the device: proof `i` against the preprocessed traces
+    /// `preps[program_of[i]]`.  One verdict per proof, each exactly what `verify_bytes` returns for that proof alone.
+    pub fn verify_batch_bytes(&mut self, proofs: &[&[u8]], preps: &[[MatrixView<'_>; 2]], program_of: &[u32], repr: Repr) -> Result<Vec<Verdict>> {
+        assert_eq!(proofs.len(), program_of.len(), "one program index per proof");
+        let prep_raw: Vec<vgpu_matrix> = preps.iter().flat_map(|p| p.iter().map(MatrixView::raw)).collect();
+        let ptrs: Vec<*const u8> = proofs.iter().map(|p| p.as_ptr()).collect();
+        let lens: Vec<u64> = proofs.iter().map(|p| p.len() as u64).collect();
+        let mut verdicts = vec![-1i32; proofs.len()];
+        let code = unsafe {
+            sys::vgpu_verify_batch(self.raw, ptrs.as_ptr(), lens.as_ptr(), proofs.len() as u32, prep_raw.as_ptr(), preps.len() as u32,
+                                   program_of.as_ptr(), repr.raw(), verdicts.as_mut_ptr())
+        };
+        self.check(code)?;
+        Ok(verdicts.into_iter().map(|v| if v == sys::VGPU_ACCEPT { Verdict::Accept } else { Verdict::Reject(v) }).collect())
+    }
+
     /// Kernels launched by this context so far.
     pub fn launch_count(&self) -> u64 {
         unsafe { sys::vgpu_ctx_launch_count(self.raw) }

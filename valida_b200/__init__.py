@@ -16,6 +16,8 @@ from .api import (  # noqa: F401
     StarkConfig,
     prove_machine,
     verify_machine,
+    verify_machines,
+    last_verify_batch_phases,
     VerificationError,
     last_prove_phases,
     fib_program,

@@ -77,6 +77,9 @@ def _load():
         "vgpu_tree_share": (None, [u64, C.c_int32, C.c_int32, C.POINTER(u64), C.POINTER(u64), C.POINTER(C.c_int32)]),
         "vgpu_open": (C.c_int32, [vp, C.POINTER(vp), C.c_uint32, u32p, u32p, C.POINTER(C.POINTER(C.c_uint8)), C.POINTER(u64)]),
         "vgpu_verify": (C.c_int32, [vp, C.c_char_p, u64, C.POINTER(_Matrix), C.c_int32, C.POINTER(C.c_int32)]),
+        "vgpu_verify_batch": (C.c_int32, [vp, C.POINTER(C.c_char_p), C.POINTER(u64), C.c_uint32, C.POINTER(_Matrix), C.c_uint32, u32p, C.c_int32,
+                                          C.POINTER(C.c_int32)]),
+        "vgpu_last_verify_batch_phases": (C.c_uint32, [vp, C.POINTER(C.c_char_p), C.POINTER(C.c_float), C.c_uint32]),
         "vgpu_prove": (C.c_int32, [vp, C.POINTER(_Matrix), C.POINTER(_Matrix), C.c_int32, C.POINTER(C.POINTER(C.c_uint8)), C.POINTER(u64)]),
         "vgpu_prove_device": (C.c_int32, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(C.POINTER(C.c_uint8)), C.POINTER(u64)]),
         "vgpu_free_bytes": (None, [C.POINTER(C.c_uint8)]),
@@ -511,6 +514,37 @@ def verify_machine(config, proof, preprocessed):
     ctx.check(lib().vgpu_verify(ctx._h, bytes(proof), len(proof), b, REPR_CANONICAL, C.byref(verdict)))
     if verdict.value != 0:
         raise VerificationError(verdict.value)
+
+
+def verify_machines(config, proofs, preprocessed_list, program_of=None):
+    """Machine::verify for many proofs in one call, checked on the device (vgpu_verify_batch).  Returns one verdict per proof:
+    0 = accepted, otherwise the VGPU_REJECT_* code vgpu_verify gives that proof alone (no exception for a rejected proof).
+
+    proofs: CBOR bytes; preprocessed_list: one (program, range) pair of row-major canonical traces per program;
+    program_of[i]: the index in preprocessed_list of proof i's program (default: preprocessed_list[i])."""
+    ctx = config.ctx
+    n = len(proofs)
+    if program_of is None:
+        program_of = list(range(n))
+    if len(program_of) != n:
+        raise ValueError("program_of needs one entry per proof")
+    keep = [_as_u32(m) for pair in preprocessed_list for m in pair]
+    mats = (_Matrix * max(1, len(keep)))(*[_mat(m) for m in keep])
+    blobs = [bytes(p) for p in proofs]
+    ptrs = (C.c_char_p * max(1, n))(*blobs)
+    lens = (C.c_uint64 * max(1, n))(*[len(p) for p in blobs])
+    prog = (C.c_uint32 * max(1, n))(*[int(g) for g in program_of])
+    verdicts = (C.c_int32 * max(1, n))()
+    ctx.check(lib().vgpu_verify_batch(ctx._h, ptrs, lens, n, mats, len(preprocessed_list), prog, REPR_CANONICAL, verdicts))
+    return [int(verdicts[i]) for i in range(n)]
+
+
+def last_verify_batch_phases(ctx):
+    """[(stretch, wall-clock ms)] of the last verify_machines call on ctx: decode, commitments, transcripts, packing, device."""
+    names = (C.c_char_p * 16)()
+    ms = (C.c_float * 16)()
+    n = lib().vgpu_last_verify_batch_phases(ctx._h, names, ms, 16)
+    return [(names[i].decode(), float(ms[i])) for i in range(min(n, 16))]
 
 
 def last_prove_phases(ctx):

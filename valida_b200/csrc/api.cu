@@ -172,7 +172,8 @@ uint64_t vgpu_ctx_launch_count(const vgpu_ctx* ctx) { return ctx->launches; }
 
 int32_t vgpu_ctx_set_kernel_timing(vgpu_ctx* ctx, int32_t on) { ctx->ktiming = on != 0; return 0; }
 static const char* KCLASS_NAMES[KC_COUNT] = {"ntt_pass_kernel", "leaf_hash_kernel", "compress_layer_kernel", "fri_leaf_hash_kernel", "transpose (rm<->cm)",
-                                             "perm trace kernels", "quotient_kernel", "inverse denominators", "bary_kernel", "reduced_opening_kernel", "fri_fold_kernel", "peer-store exchange", "all-gathers + barriers (incl. waiting for the slowest rank)", "other"};
+                                             "perm trace kernels", "quotient_kernel", "inverse denominators", "bary_kernel", "reduced_opening_kernel", "fri_fold_kernel", "peer-store exchange", "all-gathers + barriers (incl. waiting for the slowest rank)", "other",
+                                             "verify_merkle_kernel", "verify_open_kernel", "verify_fold_kernel", "verify_constraints_kernel"};
 uint32_t vgpu_ctx_kernel_stats(vgpu_ctx* ctx, const char** names, uint32_t* launches, float* ms, double* bytes, uint32_t cap) {
     cudaStreamSynchronize(ctx->stream);
     uint32_t n[KC_COUNT] = {0}; float t[KC_COUNT] = {0}; double b[KC_COUNT] = {0};

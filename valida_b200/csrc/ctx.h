@@ -22,7 +22,8 @@ struct PowTable {            // device tables of Montgomery words
 };
 
 // kernel classes for the optional per-launch CUDA-event timing (bench.py's roofline line)
-enum KClass { KC_NTT = 0, KC_LEAF_HASH, KC_COMPRESS, KC_FRI_LEAF, KC_TRANSPOSE, KC_PERM, KC_QUOTIENT, KC_INVDEN, KC_BARY, KC_REDUCED_OPENING, KC_FRI_FOLD, KC_EXCHANGE, KC_COLLECTIVE, KC_OTHER, KC_COUNT };
+enum KClass { KC_NTT = 0, KC_LEAF_HASH, KC_COMPRESS, KC_FRI_LEAF, KC_TRANSPOSE, KC_PERM, KC_QUOTIENT, KC_INVDEN, KC_BARY, KC_REDUCED_OPENING, KC_FRI_FOLD, KC_EXCHANGE, KC_COLLECTIVE, KC_OTHER,
+             KC_VERIFY_MERKLE, KC_VERIFY_OPEN, KC_VERIFY_FOLD, KC_VERIFY_CONSTRAINTS, KC_COUNT };
 struct KTimer { cudaEvent_t a, b; int cls; double bytes; };
 
 struct vgpu_ctx {
@@ -49,6 +50,7 @@ struct vgpu_ctx {
     std::vector<PhaseMark> phase_marks;                         // event pairs of the last prove (read by vgpu_last_prove_phases)
     std::vector<std::pair<const char*, float>> host_phases;     // host-side stretches of the last prove (wall clock)
     bool in_host_prove = false;
+    std::vector<std::pair<const char*, float>> verify_phases;   // host / device stretches of the last vgpu_verify_batch (wall clock)
     // size-keyed cache of device buffers: a proof repeats the same allocation sizes every step, so after the
     // first step no driver allocator call is made (single stream => reuse in enqueue order is safe)
     std::multimap<size_t, void*> free_bufs;

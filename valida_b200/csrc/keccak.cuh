@@ -5,6 +5,7 @@
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
+#include "bb.cuh"
 
 namespace kk {
 
@@ -113,5 +114,58 @@ __device__ __forceinline__ void keccak_f_peeled(uint2 A[25]) {
     if (LAST) keccak_round(A, make_uint2(0x80008008u, 0x80000000u));
 }
 __device__ __forceinline__ void keccak_f(uint2 A[25]) { keccak_f_peeled<false, false>(A); }
+
+// ---- SerializingHasher32<Keccak256Hash> and CompressionFunctionFromHasher<_, _, 2, 8> over canonical words (the Merkle trees of
+// merkle.cu and the paths the batch verifier walks in verify_batch.cu) ------------------------------------------------------------------
+constexpr int RATE_WORDS = 34;   // 136-byte rate
+
+// Sponge over `nwords` canonical words fetched by `fetch(i)`; Keccak pad 0x01 .. 0x80.
+template <bool SHORT = false, class Fetch>
+__device__ __forceinline__ void keccak256_words(const uint32_t nwords, Fetch fetch, uint32_t out[8]) {
+    uint2 A[25];
+#pragma unroll
+    for (int i = 0; i < 25; i++) A[i] = make_uint2(0, 0);
+    uint32_t nblocks = nwords / RATE_WORDS + 1;
+    if (SHORT) {   // a single block whose length the compiler sees (64-byte compression, FRI leaf): zero lanes fold away in round 0
+#pragma unroll
+        for (int i = 0; i < RATE_WORDS / 2; i++) {
+            const uint32_t g0 = 2 * i, g1 = g0 + 1;
+            uint32_t w0 = g0 < nwords ? fetch(g0) : (g0 == nwords ? 1u : 0u);
+            uint32_t w1 = g1 < nwords ? fetch(g1) : (g1 == nwords ? 1u : 0u);
+            if (i == RATE_WORDS / 2 - 1) w1 ^= 0x80000000u;
+            A[i] = make_uint2(w0, w1);
+        }
+        kk::keccak_f_peeled<true, true>(A);
+        out[0] = A[0].x; out[1] = A[0].y; out[2] = A[1].x; out[3] = A[1].y;
+        out[4] = A[2].x; out[5] = A[2].y; out[6] = A[3].x; out[7] = A[3].y;
+        return;
+    }
+    for (uint32_t b = 0; b < nblocks; b++) {
+        uint32_t base = b * RATE_WORDS;
+#pragma unroll
+        for (int i = 0; i < RATE_WORDS / 2; i++) {
+            uint32_t g0 = base + 2 * i, g1 = g0 + 1;
+            uint32_t w0 = g0 < nwords ? fetch(g0) : (g0 == nwords ? 1u : 0u);
+            uint32_t w1 = g1 < nwords ? fetch(g1) : (g1 == nwords ? 1u : 0u);
+            if (i == RATE_WORDS / 2 - 1 && b == nblocks - 1) w1 ^= 0x80000000u;
+            A[i].x ^= w0; A[i].y ^= w1;
+        }
+        if (b == nblocks - 1) kk::keccak_f_peeled<false, true>(A); else kk::keccak_f(A);
+    }
+    out[0] = A[0].x; out[1] = A[0].y; out[2] = A[1].x; out[3] = A[1].y;
+    out[4] = A[2].x; out[5] = A[2].y; out[6] = A[3].x; out[7] = A[3].y;
+}
+
+__device__ __forceinline__ uint32_t wrap_mod_p(uint32_t w) {   // F::from_wrapped_u32
+    w = bb::umin32(w, w - bb::P);
+    return bb::umin32(w, w - bb::P);
+}
+
+__device__ __forceinline__ void compress_pair(const uint32_t l[8], const uint32_t r[8], uint32_t out[8]) {
+    uint32_t d[8];
+    keccak256_words<true>(16, [&](uint32_t i) { return i < 8 ? l[i] : r[i - 8]; }, d);
+#pragma unroll
+    for (int i = 0; i < 8; i++) out[i] = wrap_mod_p(d[i]);
+}
 
 }  // namespace kk

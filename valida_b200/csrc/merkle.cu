@@ -20,49 +20,9 @@
 
 namespace {
 
-constexpr int RATE_WORDS = 34;   // 136-byte rate
-
-// Sponge over `nwords` canonical words fetched by `fetch(i)`; Keccak pad 0x01 .. 0x80.
-template <bool SHORT = false, class Fetch>
-__device__ __forceinline__ void keccak256_words(const uint32_t nwords, Fetch fetch, uint32_t out[8]) {
-    uint2 A[25];
-#pragma unroll
-    for (int i = 0; i < 25; i++) A[i] = make_uint2(0, 0);
-    uint32_t nblocks = nwords / RATE_WORDS + 1;
-    if (SHORT) {   // a single block whose length the compiler sees (64-byte compression, FRI leaf): zero lanes fold away in round 0
-#pragma unroll
-        for (int i = 0; i < RATE_WORDS / 2; i++) {
-            const uint32_t g0 = 2 * i, g1 = g0 + 1;
-            uint32_t w0 = g0 < nwords ? fetch(g0) : (g0 == nwords ? 1u : 0u);
-            uint32_t w1 = g1 < nwords ? fetch(g1) : (g1 == nwords ? 1u : 0u);
-            if (i == RATE_WORDS / 2 - 1) w1 ^= 0x80000000u;
-            A[i] = make_uint2(w0, w1);
-        }
-        kk::keccak_f_peeled<true, true>(A);
-        out[0] = A[0].x; out[1] = A[0].y; out[2] = A[1].x; out[3] = A[1].y;
-        out[4] = A[2].x; out[5] = A[2].y; out[6] = A[3].x; out[7] = A[3].y;
-        return;
-    }
-    for (uint32_t b = 0; b < nblocks; b++) {
-        uint32_t base = b * RATE_WORDS;
-#pragma unroll
-        for (int i = 0; i < RATE_WORDS / 2; i++) {
-            uint32_t g0 = base + 2 * i, g1 = g0 + 1;
-            uint32_t w0 = g0 < nwords ? fetch(g0) : (g0 == nwords ? 1u : 0u);
-            uint32_t w1 = g1 < nwords ? fetch(g1) : (g1 == nwords ? 1u : 0u);
-            if (i == RATE_WORDS / 2 - 1 && b == nblocks - 1) w1 ^= 0x80000000u;
-            A[i].x ^= w0; A[i].y ^= w1;
-        }
-        if (b == nblocks - 1) kk::keccak_f_peeled<false, true>(A); else kk::keccak_f(A);
-    }
-    out[0] = A[0].x; out[1] = A[0].y; out[2] = A[1].x; out[3] = A[1].y;
-    out[4] = A[2].x; out[5] = A[2].y; out[6] = A[3].x; out[7] = A[3].y;
-}
-
-__device__ __forceinline__ uint32_t wrap_mod_p(uint32_t w) {   // F::from_wrapped_u32
-    w = bb::umin32(w, w - bb::P);
-    return bb::umin32(w, w - bb::P);
-}
+using kk::keccak256_words;
+using kk::wrap_mod_p;
+using kk::compress_pair;
 
 // colptr[i] = device pointer to column i of the concatenated row (all matrices of this height).
 // rows [row0, row0 + nrows) of the layer (a rank's share when the tree is split across GPUs)
@@ -75,13 +35,6 @@ __global__ void __launch_bounds__(128) leaf_hash_kernel(const uint32_t* const* _
     uint4* o = reinterpret_cast<uint4*>(digests + r * 8);
     o[0] = make_uint4(wrap_mod_p(d[0]), wrap_mod_p(d[1]), wrap_mod_p(d[2]), wrap_mod_p(d[3]));
     o[1] = make_uint4(wrap_mod_p(d[4]), wrap_mod_p(d[5]), wrap_mod_p(d[6]), wrap_mod_p(d[7]));
-}
-
-__device__ __forceinline__ void compress_pair(const uint32_t l[8], const uint32_t r[8], uint32_t out[8]) {
-    uint32_t d[8];
-    keccak256_words<true>(16, [&](uint32_t i) { return i < 8 ? l[i] : r[i - 8]; }, d);
-#pragma unroll
-    for (int i = 0; i < 8; i++) out[i] = wrap_mod_p(d[i]);
 }
 
 // next[i] = compress(prev[2i], prev[2i+1]) ; if inject != null: next[i] = compress(next[i], inject[i])

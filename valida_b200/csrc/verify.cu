@@ -1,113 +1,23 @@
-// Out-of-domain constraint check of ONE chip — the verifier's half of the AIR.
-// Replaces verify_constraints (machine/src/verify.rs:11-107) with its VerifierConstraintFolder
-// (machine/src/folding_builder.rs:127-220): the opened trace / permutation / quotient values at zeta
-// are pushed through the SAME Air::eval text the device quotient sweep uses (airs.cuh, value type X =
-// degree-5 extension) and through eval_permutation_constraints (machine/src/chip.rs:210-289); the folded
-// sum must equal Z_H(zeta) * quotient(zeta).  Host code (a few hundred extension multiplications per
-// chip); it lives in a .cu file only because it instantiates the BB_HD templates of airs.cuh.
+// Out-of-domain constraint check of ONE chip — the verifier's half of the AIR — for vgpu_verify.
+// The folding itself is verify_chip.cuh (shared with the batch verifier's constraint kernel); this wrapper checks the counts of
+// the opened values and folds the LogUp randomness into the chip description.  Host code (a few hundred extension
+// multiplications per chip); it lives in a .cu file only because it instantiates the BB_HD templates of airs.cuh.
 #include "ctx.h"
 #include "devchip.h"
-#include "airs.cuh"
+#include "verify_chip.cuh"
 #include "verify.h"
 
-namespace {
-
-using bb::E5;
-using air::X;
-
-struct VerifierFolder {
-    using V = X;
-    const E5* lrow; const E5* nrow;
-    X first, last, trans;
-    E5 alpha, acc;
-    X L(int c) const { return X{lrow[c]}; }
-    X N(int c) const { return X{nrow[c]}; }
-    void z(const X& x) { acc = bb::e5_add(bb::e5_mul(acc, alpha), x.e); }   // Horner, folding_builder.rs:196-200
-    void z_ext(const E5& x) { acc = bb::e5_add(bb::e5_mul(acc, alpha), x); }
-};
-
-template <int CHIP> void eval_one(VerifierFolder& f) { air::eval_chip<CHIP>(f); }
-
-void eval_air(uint32_t chip_id, VerifierFolder& f) {
-    switch (chip_id) {
-        case 0: eval_one<0>(f); break;   case 3: eval_one<3>(f); break;   case 4: eval_one<4>(f); break;
-        case 5: eval_one<5>(f); break;   case 7: eval_one<7>(f); break;   case 8: eval_one<8>(f); break;
-        case 9: eval_one<9>(f); break;   case 10: eval_one<10>(f); break; case 11: eval_one<11>(f); break;
-        case 13: eval_one<13>(f); break; default: break;   // program, memory, div, range: empty eval
-    }
-}
-
-// VirtualPairCol::apply over extension-valued rows (p3_air::VirtualPairCol; machine/src/chip.rs:76-80)
-bool pair_col_ext(const DevPairCol& pc, const E5* main_row, E5* out) {
-    E5 v = bb::e5_from_base(pc.constant);
-    for (uint32_t t = 0; t < pc.n_terms; t++) {
-        if (pc.is_prep[t]) return false;   // the reference never opens the preprocessed commitment (derive/src/lib.rs:379-392)
-        v = bb::e5_add(v, bb::e5_mul_base(main_row[pc.column[t]], pc.weight[t]));
-    }
-    *out = v;
-    return true;
-}
-
-// sum_l v[5m + l] * X^l : the opened flattened columns of one extension column back to one extension value
-E5 unflatten(const E5* v, uint32_t m) {
-    E5 s = bb::e5_zero();
-    for (int l = 0; l < 5; l++) {
-        E5 mono = bb::e5_zero();
-        mono.c[l] = bb::R1;
-        s = bb::e5_add(s, bb::e5_mul(v[5 * m + l], mono));
-    }
-    return s;
-}
-
-}  // namespace
-
 int32_t vg_verify_chip_constraints(vgpu_ctx* ctx, const vgpu_chip_desc* chip, uint32_t log_degree, const VgChipOpening& ov,
-                                   const E5& cumulative_sum, const E5& zeta, const E5& alpha, const uint32_t perm_challenges[15], bool* ok) {
+                                   const bb::E5& cumulative_sum, const bb::E5& zeta, const bb::E5& alpha, const uint32_t perm_challenges[15], bool* ok) {
     *ok = false;
-    const uint32_t k = chip->n_interactions, pw = k + 1;
+    const uint32_t pw = chip->n_interactions + 1;
     if (ov.trace_local.size() != chip->width || ov.trace_next.size() != chip->width) return 0;
     if (ov.perm_local.size() != 5 * pw || ov.perm_next.size() != 5 * pw || ov.quotient_chunks.size() != 10) return 0;
     DevChip dc;
     VG_TRY(vg_build_devchip(ctx, chip, perm_challenges, &dc));
-    const uint32_t g_inv = bb::inv(bb::two_adic_generator_monty((int)log_degree));
-    const E5 z_h = bb::e5_sub_base(bb::e5_exp_pow2(zeta, (int)log_degree), bb::R1);
-    const E5 zm1 = bb::e5_sub_base(zeta, bb::R1), zmg = bb::e5_sub_base(zeta, g_inv);
-    if (bb::e5_is_zero(zm1) || bb::e5_is_zero(zmg)) return 0;
-    VerifierFolder f;
-    f.lrow = ov.trace_local.data(); f.nrow = ov.trace_next.data();
-    f.first = X{bb::e5_mul(z_h, bb::e5_inv(zm1))};
-    f.last = X{bb::e5_mul(z_h, bb::e5_inv(zmg))};
-    f.trans = X{zmg};
-    f.alpha = alpha; f.acc = bb::e5_zero();
-    eval_air(chip->chip_id, f);
-    {   // eval_permutation_constraints
-        std::vector<E5> pl(pw), pn(pw);
-        for (uint32_t m = 0; m < pw; m++) { pl[m] = unflatten(ov.perm_local.data(), m); pn[m] = unflatten(ov.perm_next.data(), m); }
-        E5 rhs = bb::e5_zero(), phi0 = bb::e5_zero();
-        for (uint32_t m = 0; m < k; m++) {
-            const DevInteraction& it = dc.interactions[m];
-            E5 rlc = it.alpha;
-            for (uint32_t j = 0; j < it.n_fields; j++) {
-                E5 e;
-                if (!pair_col_ext(it.fields[j], f.lrow, &e)) VG_FAIL(ctx, "verify: interaction reads a preprocessed column, which the proof does not open");
-                rlc = bb::e5_add(rlc, bb::e5_mul(dc.betas[j], e));
-            }
-            f.z_ext(bb::e5_sub_base(bb::e5_mul(rlc, pl[m]), bb::R1));
-            E5 mult_l, mult_n;
-            if (!pair_col_ext(it.count, f.lrow, &mult_l) || !pair_col_ext(it.count, f.nrow, &mult_n)) VG_FAIL(ctx, "verify: interaction count reads a preprocessed column");
-            const E5 tl = bb::e5_mul(pl[m], mult_l), tn = bb::e5_mul(pn[m], mult_n);
-            if (it.is_send) { phi0 = bb::e5_add(phi0, tl); rhs = bb::e5_add(rhs, tn); }
-            else { phi0 = bb::e5_sub(phi0, tl); rhs = bb::e5_sub(rhs, tn); }
-        }
-        f.z_ext(bb::e5_mul(f.trans.e, bb::e5_sub(bb::e5_sub(pn[k], pl[k]), rhs)));
-        f.z_ext(bb::e5_mul(f.first.e, bb::e5_sub(pl[k], phi0)));
-        f.z_ext(bb::e5_mul(f.last.e, bb::e5_sub(pl[k], cumulative_sum)));
-    }
-    // quotient(zeta) = chunk_0(zeta^2) + zeta * chunk_1(zeta^2)   (log_quotient_degree = 1)
-    const E5 quot = bb::e5_add(unflatten(ov.quotient_chunks.data(), 0), bb::e5_mul(unflatten(ov.quotient_chunks.data(), 1), zeta));
-    const E5 want = bb::e5_mul(z_h, quot);
-    bool same = true;
-    for (int l = 0; l < 5; l++) same = same && (want.c[l] == f.acc.c[l]);
-    *ok = same;
+    const vchip::ChipOpenedView view{ov.trace_local.data(), ov.trace_next.data(), ov.perm_local.data(), ov.perm_next.data(), ov.quotient_chunks.data()};
+    const int r = vchip::chip_constraints_any(dc, log_degree, view, cumulative_sum, zeta, alpha);
+    if (r == vchip::CHIP_READS_PREPROCESSED) VG_FAIL(ctx, "verify: an interaction reads a preprocessed column, which the proof does not open");
+    *ok = r == vchip::CHIP_ACCEPT;
     return 0;
 }
